@@ -82,7 +82,12 @@ def parse():
   ap.add_argument("--exchange", default=None, choices=["direct", "peer", "nccl"],
                   help="exchange of the sharded step: 'direct' = device-driven (fixed window regions, directional flags, no host "
                        "round trip), 'peer' = host-driven NVLink peer windows with flag barriers, 'nccl' = NCCL all-to-all")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, fixed seeded "
+                       "samples, see dump_outputs) so that two builds can be compared output for output; c2 / c3 only")
   args = ap.parse_args()
+  if args.dump_outputs and (args.impl == "reference" or args.workload in ("c4", "c5")):
+    ap.error("--dump-outputs applies to the GPU step of workloads c2 and c3")
   global DIM, SLOTS
   if args.workload == "c3":
     DIM, SLOTS = 16, 26
@@ -514,6 +519,30 @@ class Tower:
     return loss.detach(), gx
 
 
+DUMP_ROWS = 1 << 17
+
+
+def dump_outputs(out_dir, table, pooled, fids, world, rank):
+  """Writes what the last timed step gave its caller: `pooled.npy`, a fixed sample of DUMP_ROWS rows of the forward's
+  pooled output, and `embeddings.npy` / `adagrad_accumulators.npy`, the table rows the backward left behind for a
+  fixed sample of DUMP_ROWS / 2 of the step's unique FIDs that this rank owns (both sorted by position / FID).  The
+  samples depend only on the batch, which is seeded, so the same arguments dump the same positions on every build.
+  c2: 16 + 8 + 8 MB."""
+  import torch
+  torch.cuda.synchronize()
+  dev = pooled.device
+  rng = np.random.default_rng(0)
+  rows = np.sort(rng.choice(pooled.shape[0], min(pooled.shape[0], DUMP_ROWS), replace=False))
+  own = np.unique(fids)
+  own = own[own % world == rank]
+  ids = np.sort(rng.choice(own, min(own.size, DUMP_ROWS // 2), replace=False))
+  ent = table.lookup_entry("item", torch.from_numpy(ids).to(dev))
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "pooled.npy"), pooled[torch.from_numpy(rows).to(dev)].cpu().numpy())
+  np.save(os.path.join(out_dir, "embeddings.npy"), ent["num"].cpu().numpy())
+  np.save(os.path.join(out_dir, "adagrad_accumulators.npy"), ent["opt"].cpu().numpy())
+
+
 def run_ours(args):
   import torch
   import torch.distributed as dist
@@ -638,6 +667,8 @@ def run_ours(args):
 
   with Clocks(local) as clk:
     ms, launches, regions = timed(dev_step, args.steps, args.warmup, args.repeats)
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, table, pooled, batches_np[(counter[0] - 1) % NB], world, rank)
   ab = {}
   if args.ab:
     _l = lib

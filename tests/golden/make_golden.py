@@ -9,7 +9,7 @@ Two kinds of vectors:
     (oracle/_ref/libmonoref.so, built by oracle/Makefile from /root/reference in place):
     runtime/hash_table/optimizer/avx_utils.h (Adagrad) and
     data/kernels/internal/uniq_hashtable.h (first-occurrence dedup ordinals).
-    -> tests/golden/ref_adagrad.npz, tests/golden/ref_uniq_fid.npz
+    -> tests/golden/ref_adagrad.npz, tests/golden/ref_adagrad_avx_lanes.npz, tests/golden/ref_uniq_fid.npz
 
 Run from the repo root in the build container (needs /root/reference):
     make -C oracle && python tests/golden/make_golden.py
@@ -202,6 +202,25 @@ def main():
     cases[f"c{ci}_norm"] = np.stack(seq_norm)
   cases["n_cases"] = np.int64(8)
   np.savez(os.path.join(HERE, "ref_adagrad.npz"), **cases)
+
+  # rows whose every lane takes the AVX path (dim % 8 == 0): the oracle must match these bit for bit over the whole row
+  rng = np.random.default_rng(1)
+  lr = np.float32(0.01)
+  lanes = {"lr": lr}
+  for ci, dim in enumerate((8, 24, 64)):
+    num, norm = rng.standard_normal(dim).astype(np.float32), np.full(dim, 0.1, np.float32)
+    lanes[f"c{ci}_num0"], lanes[f"c{ci}_norm0"] = num.copy(), norm.copy()
+    seq_num, seq_norm, grads = [], [], []
+    for step in range(5):
+      g = rng.standard_normal(dim).astype(np.float32)
+      ref.ref_adagrad(num.ctypes.data_as(C.c_void_p), norm.ctypes.data_as(C.c_void_p),
+                      g.ctypes.data_as(C.c_void_p), C.c_int64(dim), C.c_float(lr), C.c_float(0.0))
+      grads.append(g.copy()); seq_num.append(num.copy()); seq_norm.append(norm.copy())
+    lanes[f"c{ci}_grads"] = np.stack(grads)
+    lanes[f"c{ci}_num"] = np.stack(seq_num)
+    lanes[f"c{ci}_norm"] = np.stack(seq_norm)
+  lanes["n_cases"] = np.int64(3)
+  np.savez(os.path.join(HERE, "ref_adagrad_avx_lanes.npz"), **lanes)
 
   # first-occurrence ordinals from the reference's MultiShardUniqHashTable
   u = {}

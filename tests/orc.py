@@ -9,7 +9,6 @@ from monolith_b200.entry import to_c_table_cfgs
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 _so = None
-_ref = None
 
 
 def lib():
@@ -25,15 +24,6 @@ def lib():
     _so.orc_uniform_init.argtypes = [C.c_uint64, C.c_int64, C.c_int, C.c_float, C.c_float]
     _so.orc_ps_size.restype = C.c_int64
   return _so
-
-
-def ref():
-  """oracle/_ref: the real reference headers compiled in place (None when not built)."""
-  global _ref
-  p = os.path.join(ROOT, "oracle", "_ref", "libmonoref.so")
-  if _ref is None and os.path.exists(p):
-    _ref = C.CDLL(p)
-  return _ref
 
 
 def p(a):

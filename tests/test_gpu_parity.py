@@ -1196,6 +1196,32 @@ def test_bench_shape_step_vs_oracle(dev):
   assert float((np.abs(got[~cold][:, :-2] - want[~cold][:, :-2]) / scale).max()) < 2e-3
 
 
+def test_bench_dump_outputs_follow_the_step_count(tmp_path):
+  """bench.py --dump-outputs writes the last timed step's outputs as float32 arrays.  With one timed region the bench
+  runs warmup + steps steps over 4 rotating batches: warmup 2 + 1 step dumps bit for bit what warmup 1 + 2 steps dumps
+  (another process, same inputs), and warmup 1 + 6 steps ends on the same batch after four more Adagrad updates."""
+  import subprocess
+  import sys
+  root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+  def run(name, steps, warmup):
+    out = tmp_path / name
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--keys", "200000", "--batch", "8192",
+                        "--steps", str(steps), "--warmup", str(warmup), "--repeats", "1", "--no-parity", "--no-e2e",
+                        "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, timeout=600, cwd=root)
+    assert r.returncode == 0, r.stderr[-2000:]
+    return {k: np.load(out / f"{k}.npy") for k in ("pooled", "embeddings", "adagrad_accumulators")}
+
+  a, b, c = run("a", 2, 1), run("b", 1, 2), run("c", 6, 1)
+  assert a["pooled"].shape == (8192 * 2, 32) and a["embeddings"].shape == a["adagrad_accumulators"].shape
+  assert all(v.dtype == np.float32 for v in a.values()) and a["embeddings"].shape[0] > 1000
+  for k in a:
+    np.testing.assert_array_equal(a[k].view(np.uint32), b[k].view(np.uint32))
+  assert (c["adagrad_accumulators"] >= a["adagrad_accumulators"]).all()
+  assert (c["adagrad_accumulators"] > a["adagrad_accumulators"]).any()
+
+
 def test_two_host_threads_share_one_handle(dev):
   """Two host threads drive ONE table handle concurrently (lookups against updates of disjoint FID sets, each on its
   own stream): the per-handle lock of the C ABI serialises them; results equal the sequential ones (ref: TF runs the

@@ -174,21 +174,17 @@ def test_first_occurrence_ordinals_vs_reference_uniq_hashtable_fixture():
     assert (offs - base[shard]).tolist() == z[f"c{ci}_uniq_idx"].tolist()
 
 
-def test_live_ref_library_if_present():
-  """When oracle/_ref is built (build container), compare fresh random vectors too."""
-  ref = orc.ref()
-  if ref is None:
-    pytest.skip("oracle/_ref not built here")
+def test_adagrad_avx_lanes_bit_exact_vs_reference_header_fixture():
+  """Rows of 8, 24 and 64 floats (every lane on the AVX path of avx_utils.h), unit-normal state and gradients, lr 0.01:
+  the oracle's Adagrad equals the reference header's bit for bit after every one of five steps."""
   import ctypes as C
-  rng = np.random.default_rng(1)
-  for dim in (8, 24, 64):
-    a, an = rng.standard_normal(dim).astype(np.float32), np.full(dim, 0.1, np.float32)
-    b, bn = a.copy(), an.copy()
-    for _ in range(5):
-      g = rng.standard_normal(dim).astype(np.float32)
-      ref.ref_adagrad(orc.p(a), orc.p(an), orc.p(g), C.c_int64(dim), C.c_float(0.01), C.c_float(0.0))
-      orc.lib().orc_adagrad(orc.p(b), orc.p(bn), orc.p(g), C.c_int64(dim), C.c_float(0.01), C.c_float(0.0))
-    assert np.array_equal(a, b) and np.array_equal(an, bn)
+  z = np.load(os.path.join(G, "ref_adagrad_avx_lanes.npz"))
+  for ci in range(int(z["n_cases"])):
+    num, norm = z[f"c{ci}_num0"].copy(), z[f"c{ci}_norm0"].copy()
+    for step in range(z[f"c{ci}_grads"].shape[0]):
+      g = np.ascontiguousarray(z[f"c{ci}_grads"][step])
+      orc.lib().orc_adagrad(orc.p(num), orc.p(norm), orc.p(g), C.c_int64(num.size), C.c_float(z["lr"]), C.c_float(0.0))
+      assert np.array_equal(num, z[f"c{ci}_num"][step]) and np.array_equal(norm, z[f"c{ci}_norm"][step]), (ci, step)
 
 
 def test_layout_pooling_vs_reference_numpy_oracle_fixture():
